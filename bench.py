@@ -1,11 +1,13 @@
 #!/usr/bin/env python
 """bench.py -- sorted-KV GB/s of the Tez shuffle sort/merge hot path on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 N=1 workload = BASELINE config 2: 1e8 records, 16 B key / 64 B value, 64 partitions (HashPartitioner,
 TezBytesComparator) -> file.out bytes bit-identical to the reference format.  A "step" is one complete pass of the
-hot path over that batch (partition + sort + IFile emit with CRC).
+hot path over that batch (partition + sort + IFile emit with CRC); every GPU leg of the N=1 run times K steps.
+--dump-outputs DIR (N=1): writes what the last timed step returned as DIR/*.npy (see dump_outputs), so that two builds
+can be compared output for output; the inputs are the same seeded records in every run.
   value   : KV payload GB/s with the records already resident in HBM (device-timed, CUDA events on the library stream)
   e2e     : the same metric through the C ABI with HOST buffers (H2D of the records and D2H of file.out inside the
             timed region) -- the call a Tez task makes
@@ -236,6 +238,35 @@ def load_traffic():
     return None
 
 
+def dump_outputs(out_dir, d_out, out_len, index, chunks=2048, chunk_bytes=4096, seed=0):
+    """What one sort_device_fixed call hands its caller, as float arrays (about 34 MB in all):
+      index.npy                  (P, 3) float64: segment start, raw length, part length of every partition
+      file_out_len.npy           (1,) float64: bytes of file.out
+      segment_crc32.npy          (P,) float64: every segment's CRC32 trailer (covers all of its bytes; -1 = no segment)
+      file_out_sample.npy        (chunks, chunk_bytes) float32: file.out bytes at seeded offsets
+      file_out_sample_offsets.npy (chunks,) float64: those offsets
+    The offsets depend only on `seed` and the output length, so equal outputs give equal files."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    out = d_out[:out_len]
+    index = np.asarray(index, dtype=np.int64)
+    crc = np.full(len(index), -1.0)
+    has = index[:, 2] > 0
+    if has.any():
+        at = torch.from_numpy(index[has, 0] + index[has, 2] - 4)[:, None] + torch.arange(4)
+        b = out[at.to(out.device)].cpu().numpy().astype(np.uint64)
+        crc[has] = (b[:, 0] << 24) | (b[:, 1] << 16) | (b[:, 2] << 8) | b[:, 3]
+    width = min(chunk_bytes, out_len)
+    offs = np.sort(np.random.default_rng(seed).integers(0, out_len - width + 1, size=chunks))
+    at = (torch.from_numpy(offs)[:, None] + torch.arange(width)).to(out.device)
+    sample = out[at].cpu().numpy().astype(np.float32)
+    for name, a in (("index", index.astype(np.float64)), ("file_out_len", np.array([out_len], dtype=np.float64)),
+                    ("segment_crc32", crc), ("file_out_sample", sample),
+                    ("file_out_sample_offsets", offs.astype(np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def single_gpu(args):
     import torch
     import tez_b200 as T
@@ -274,6 +305,8 @@ def single_gpu(args):
     ms_step = ev0.elapsed_time(ev1) / args.steps
     value = n * REC / (ms_step * 1e-3) / 1e9
     assert out_len == n * OUT_REC + 10 * int((index[:, 1] > 0).sum())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d_out, out_len, index)
 
     peak, peak_src = hbm_peak()
     emit = sum(emit_ms) / len(emit_ms)
@@ -317,7 +350,7 @@ def single_gpu(args):
             step4()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        k4 = max(3, min(args.steps, 5))
+        k4 = args.steps
         for _ in range(k4):
             st4, mst4, mlen4, out_len4 = step4()
         torch.cuda.synchronize()
@@ -344,8 +377,7 @@ def single_gpu(args):
             h_outs = [torch.empty(cap + 4096, dtype=torch.uint8, pin_memory=True) for _ in range(slots)]
             torch.cuda.synchronize()
             sorters = [T.GpuSorter(P, fixed=(KEY_LEN, VAL_LEN), device=0) for _ in range(slots)]
-            esteps = max(slots, min(args.steps, args.e2e_steps))
-            esteps -= esteps % slots
+            esteps = args.steps
             out_bytes = [0] * slots
 
             # --e2e-direction-locks: one transfer at a time per PCIe direction (a slot's upload next to the other slot's
@@ -371,18 +403,19 @@ def single_gpu(args):
                         out, _, _, _ = s2.flush_to_memory(out=ho)
                     out_bytes[k] = int(len(out))
 
-            def run_e2e(nsteps_per_slot):
+            def run_e2e(total_steps):
                 ev = [threading.Event() for _ in range(slots + 1)]
                 ev[0].set()
-                ths = [threading.Thread(target=e2e_worker, args=(k, nsteps_per_slot, ev[k], ev[k + 1])) for k in range(slots)]
+                per_slot = [total_steps // slots + (k < total_steps % slots) for k in range(slots)]
+                ths = [threading.Thread(target=e2e_worker, args=(k, per_slot[k], ev[k], ev[k + 1])) for k in range(slots)]
                 for t in ths:
                     t.start()
                 for t in ths:
                     t.join()
 
-            run_e2e(1)  # warm-up: allocations, pinning
+            run_e2e(slots)  # warm-up: allocations, pinning
             t0 = time.perf_counter()
-            run_e2e(esteps // slots)
+            run_e2e(esteps)
             torch.cuda.synchronize()
             t = (time.perf_counter() - t0) / esteps
             e2e = {"value": round(n * REC / t / 1e9, 3), "unit": "GB/s", "h2d_bytes_per_step": n * REC,
@@ -537,7 +570,7 @@ def config3(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every GPU leg")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--records", type=int, default=None,
@@ -546,7 +579,6 @@ def main():
                     help="CPU arm: records per PipelinedSorter task (> 2^20 so that every task has two spans and its SpanMerger runs)")
     ap.add_argument("--cpu-single-records", type=int, default=10_000_000,
                     help="reference arm: records of the single-sorter sample (0 = skip)")
-    ap.add_argument("--e2e-steps", type=int, default=12)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--e2e-direction-locks", action="store_true", help="e2e leg: serialise the task slots per PCIe direction")
     ap.add_argument("--no-g1-pipeline", action="store_true")
@@ -557,8 +589,15 @@ def main():
     ap.add_argument("--c3-segments", type=int, default=256)
     ap.add_argument("--c3-segment-mb", type=int, default=64)
     ap.add_argument("--c3-cpu-segments", type=int, default=16)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="config 2 on one GPU: write the last timed step's outputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    single = args.impl != "reference" and args.config not in (1, 3, 5) and args.gpus == 1 and world == 1
+    if args.dump_outputs and not single:
+        ap.error("--dump-outputs is implemented for the single-GPU config 2 run")
     if args.records is None:
         if args.config == 5:
             args.records = 4_000_000      # 16.4 GB of records per GPU
@@ -572,7 +611,7 @@ def main():
         return config1(args)
     if args.config == 3:
         return config3(args)
-    if args.config != 5 and args.gpus == 1 and int(os.environ.get("WORLD_SIZE", "1")) == 1:
+    if single:
         return single_gpu(args)
     if args.config == 5 and "RANK" not in os.environ:      # config 5 on one GPU without torchrun: a world of one
         os.environ.update({"RANK": "0", "WORLD_SIZE": "1", "LOCAL_RANK": "0", "MASTER_ADDR": "127.0.0.1", "MASTER_PORT": "29533"})
