@@ -59,6 +59,14 @@ extern "C" {
  * depends on buffer arithmetic and thread timing: parity is then the identical index + the per-partition multiset. */
 #define TEZGPU_SORTER_UNORDERED 2
 
+/* combiner (tez.runtime.combiner.class = MRCombiner over a sum reducer; SORT/PipelinedSorter.java:601-609,815-820):
+ * the sorted records of every partition are replaced by one record per group of equal keys -- the group's key and the
+ * sum of its values, Java int / long wrap-around -- before they are written.  Combined keys are unique within a
+ * partition, so a combined segment holds no REPEAT_KEY record. */
+#define TEZGPU_COMBINE_NONE 0
+#define TEZGPU_COMBINE_INT_SUM 1    /* IntSumReducer: values are 4-byte big-endian IntWritable */
+#define TEZGPU_COMBINE_LONG_SUM 2   /* LongSumReducer (new and old API): values are 8-byte big-endian LongWritable */
+
 typedef struct tezgpu_conf {
   int32_t abi_version;                  /* TEZGPU_ABI_VERSION */
   int32_t device;                       /* CUDA ordinal */
@@ -149,6 +157,16 @@ int32_t tezgpu_sorter_sort_device_fixed(tezgpu_sorter *h, const void *d_kv, cons
 /* cudaStream_t of the handle, as an opaque pointer (so callers can record events on it) */
 void *tezgpu_sorter_stream(tezgpu_sorter *h);
 
+/* runCombineProcessor at spill time (SORT/PipelinedSorter.java:601-609): every flush writes the combined records.
+ * Call before the first collect or right after a reset; the kind stays set across resets.  TEZGPU_E_UNSUPPORTED on a
+ * TEZGPU_SORTER_UNORDERED handle; TEZGPU_E_INVALID when fixed_val_len is set and is not the kind's value width.  A
+ * collected value of the wrong width makes the flush fail with TEZGPU_E_INVALID.  With a combiner, stats.spilled_records
+ * and output_bytes_with_overhead count the combined records, output_records / output_bytes / adjacent_equal_keys /
+ * rle_used the collected ones (the RLE decision is taken before the combine). */
+int32_t tezgpu_sorter_set_combiner(tezgpu_sorter *h, int32_t kind);
+/* records into and out of the combine of the last flush (both 0 without a combiner) and its device time */
+int32_t tezgpu_sorter_combine_info(tezgpu_sorter *h, uint64_t *records_in, uint64_t *records_out, float *ms);
+
 /* ------------------------------------------------------------------------------------------------------------------
  * Merger: replaces TezMerger.merge(...) -> TezRawKeyValueIterator (SORT/TezMerger.java:717-912,
  * SORT/TezRawKeyValueIterator.java:33-87) as called from OG/MergeManager.java:804-811,899-903,1035-1041,1197-1199
@@ -210,6 +228,11 @@ int32_t tezgpu_merge_write_partitions_device(tezgpu_merger *m, void *d_out, uint
  * (SORT/PipelinedSorter.java:774-836) */
 int32_t tezgpu_merge_write_partitions(tezgpu_merger *m, const char *out_path, const char *index_path, int32_t rle,
                                       int64_t *index, tezgpu_stats *stats);
+/* combiner of a combining merge (PipelinedSorter.flush with numSpills >= tez.runtime.combine.min.spills, :815-820;
+ * MergeManager's mem->disk merges, OG/MergeManager.java:899-911): applies to the tezgpu_merge_write_* entry points;
+ * tezgpu_merge_next_batch stays the uncombined TezRawKeyValueIterator stream */
+int32_t tezgpu_merge_set_combiner(tezgpu_merger *m, int32_t kind);
+int32_t tezgpu_merge_combine_info(tezgpu_merger *m, uint64_t *records_in, uint64_t *records_out, float *ms);
 void *tezgpu_merge_stream(tezgpu_merger *m);
 int32_t tezgpu_merge_close(tezgpu_merger *m);
 

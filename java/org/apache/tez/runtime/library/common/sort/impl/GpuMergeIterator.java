@@ -78,10 +78,16 @@ public final class GpuMergeIterator implements TezRawKeyValueIterator {
 
   /** PipelinedSorter.flush's final merge: all spills, all partitions, one device pass (PipelinedSorter.java:774-836). */
   static void mergeSpillsToFile(String[] spillFiles, String[] spillIndexFiles, int partitions, int comparator,
-      boolean sendEmptyPartitionDetails, boolean checkForSameKeys, boolean writerRle, String out, String index)
-      throws IOException {
+      boolean sendEmptyPartitionDetails, boolean checkForSameKeys, boolean writerRle, int combiner, String out,
+      String index) throws IOException {
+    // combiner: GpuSorter.COMBINE_*, NONE unless numSpills >= tez.runtime.combine.min.spills (PipelinedSorter.java:815-820)
     nativeMergeSpills(spillFiles, spillIndexFiles, partitions, comparator, sendEmptyPartitionDetails, checkForSameKeys,
-        writerRle, out, index); // tezgpu_merge_open(P) + set_check_for_same_keys + tezgpu_merge_write_partitions
+        writerRle, combiner, out, index); // tezgpu_merge_open(P) + set_check_for_same_keys + set_combiner + write_partitions
+  }
+
+  /** Combiner of writeFile (a MergeManager mem->disk merge that runs the combiner, OG/MergeManager.java:899-911). */
+  void setCombiner(int kind) throws IOException {
+    nativeSetCombiner(handle, kind); // tezgpu_merge_set_combiner
   }
 
   private static native long nativeOpen(long[] addresses, long[] lengths, int[] flags, int[] partitions, int numPartitions,
@@ -91,6 +97,8 @@ public final class GpuMergeIterator implements TezRawKeyValueIterator {
   private static native boolean nativeHasMore(long h);
   private static native void nativeWriteIFile(long h, String path, boolean rle, long[] rawAndPart) throws IOException;
   private static native void nativeMergeSpills(String[] files, String[] indexFiles, int partitions, int comparator,
-      boolean sendEmpty, boolean checkForSameKeys, boolean writerRle, String out, String index) throws IOException;
+      boolean sendEmpty, boolean checkForSameKeys, boolean writerRle, int combiner, String out, String index)
+      throws IOException;
+  private static native void nativeSetCombiner(long h, int kind) throws IOException;
   private static native void nativeClose(long h);
 }

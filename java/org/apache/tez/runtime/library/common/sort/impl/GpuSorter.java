@@ -21,7 +21,9 @@ import org.apache.hadoop.io.IntWritable;
 import org.apache.hadoop.io.LongWritable;
 import org.apache.hadoop.io.RawComparator;
 import org.apache.hadoop.io.Text;
+import org.apache.tez.common.counters.TaskCounter;
 import org.apache.tez.runtime.api.OutputContext;
+import org.apache.tez.runtime.library.common.ConfigUtils;
 import org.apache.tez.runtime.library.common.comparator.TezBytesComparator;
 import org.apache.tez.runtime.library.partitioner.HashPartitioner;
 
@@ -34,6 +36,7 @@ public class GpuSorter extends ExternalSorter {
   // ids of include/tezgpu.h
   static final int CMP_BYTES = 0, CMP_TEXT = 1, CMP_BYTESWRITABLE = 2, CMP_INT = 3, CMP_LONG = 4;
   static final int PART_GIVEN = 0, PART_HASH = 1;
+  static final int COMBINE_NONE = 0, COMBINE_INT_SUM = 1, COMBINE_LONG_SUM = 2;
   private static final int BATCH_BYTES = 32 << 20;
   private static final int BATCH_RECORDS = 1 << 20;
 
@@ -46,6 +49,8 @@ public class GpuSorter extends ExternalSorter {
   private int n;
   private long collectedBytes;
   private boolean lastSpillRle;
+  private final int combineKind;
+  private final int minSpillsForCombine;
 
   private static IntBuffer direct(int ints) {
     return ByteBuffer.allocateDirect(4 * ints).order(ByteOrder.nativeOrder()).asIntBuffer();
@@ -60,6 +65,40 @@ public class GpuSorter extends ExternalSorter {
         Integer.parseInt(System.getenv().getOrDefault("TEZGPU_DEVICE", "0")));
     keySerializer.open(sink);
     valSerializer.open(sink);
+    combineKind = combinerKind(combiner, conf);
+    minSpillsForCombine = conf.getInt("tez.runtime.combine.min.spills", 3);
+    if (combineKind != COMBINE_NONE) nativeSetCombiner(handle, combineKind); // tezgpu_sorter_set_combiner
+  }
+
+  /**
+   * The combiner ExternalSorter instantiated (TezRuntimeUtils.instantiateCombiner): MRCombiner over a sum reducer runs on
+   * the device; any other combiner is not run, as before.  MRCombiner reads the reducer from mapreduce.job.combine.class
+   * under the new API and from mapred.combiner.class otherwise (ConfigUtils.useNewApi).  A sum reducer over another
+   * value class fails here instead of with a ClassCastException at the first spill.
+   */
+  static int combinerKind(Object combiner, Configuration conf) throws IOException {
+    if (combiner == null || !combiner.getClass().getName().equals("org.apache.tez.mapreduce.combine.MRCombiner")) {
+      return COMBINE_NONE;
+    }
+    final String reducer = conf.get(conf.getBoolean("mapred.mapper.new-api", false)
+        ? "mapreduce.job.combine.class" : "mapred.combiner.class", "");
+    final int kind;
+    final String need;
+    if (reducer.equals("org.apache.hadoop.mapreduce.lib.reduce.IntSumReducer")) {
+      kind = COMBINE_INT_SUM;
+      need = IntWritable.class.getName();
+    } else if (reducer.equals("org.apache.hadoop.mapreduce.lib.reduce.LongSumReducer")
+        || reducer.equals("org.apache.hadoop.mapred.lib.LongSumReducer")) {
+      kind = COMBINE_LONG_SUM;
+      need = LongWritable.class.getName();
+    } else {
+      return COMBINE_NONE;
+    }
+    final String val = ConfigUtils.getIntermediateOutputValueClass(conf).getName();
+    if (!val.equals(need)) {
+      throw new IOException("combiner " + reducer + " sums " + need + " values, but the value class is '" + val + "'");
+    }
+    return kind;
   }
 
   /** The device path supports a closed set of RawComparators; anything else keeps tez.runtime.sorter.class=PIPELINED. */
@@ -112,9 +151,16 @@ public class GpuSorter extends ExternalSorter {
     final long[] counters = new long[8];
     nativeFlush(handle, out.toString(), index.toString(), idx, counters); // tezgpu_sorter_flush: file.out + file.out.index, 0640
     nativeReset(handle);
-    lastSpillRle = counters[5] != 0;
+    lastSpillRle = counters[5] != 0;                 // decided on the records before the combine
     outputBytesWithOverheadCounter.increment(counters[0]);
-    spilledRecordsCounter.increment(counters[2]);
+    spilledRecordsCounter.increment(counters[2]);   // after the combine: what the writer wrote
+    if (combineKind != COMBINE_NONE) {
+      final long[] info = new long[2];
+      nativeCombineInfo(handle, info);              // tezgpu_sorter_combine_info
+      // counted by MRCombiner's ValuesIterator and writer in the reference
+      outputContext.getCounters().findCounter(TaskCounter.COMBINE_INPUT_RECORDS).increment(info[0]);
+      outputContext.getCounters().findCounter(TaskCounter.COMBINE_OUTPUT_RECORDS).increment(info[1]);
+    }
     if (reportPartitionStats()) {
       for (int i = 0; i < partitions; i++) partitionStats[i] += idx[3 * i + 1]; // PipelinedSorter.java:631-633
     }
@@ -138,7 +184,8 @@ public class GpuSorter extends ExternalSorter {
     finalIndexFile = mapOutputFile.getOutputIndexFileForWrite(0);
     GpuMergeIterator.mergeSpillsToFile(spillFilePaths(), spillIndexPaths(), partitions,
         comparatorId(comparator, conf), sendEmptyPartitionDetails, lastSpillRle, lastSpillRle,
-        finalOutputFile.toString(), finalIndexFile.toString());
+        numSpills >= minSpillsForCombine ? combineKind : COMBINE_NONE, finalOutputFile.toString(),
+        finalIndexFile.toString());
     numShuffleChunks.setValue(1);
   }
 
@@ -163,6 +210,9 @@ public class GpuSorter extends ExternalSorter {
    *  [4] OUTPUT_BYTES [5] rle used [6] adjacent equal keys [7] kernel launches */
   private static native void nativeFlush(long h, String out, String index, long[] idx, long[] counters) throws IOException;
   private static native void nativeReset(long h) throws IOException;
+  private static native void nativeSetCombiner(long h, int kind) throws IOException;
+  /** info: [0] records into, [1] records out of the last flush's combine */
+  private static native void nativeCombineInfo(long h, long[] info) throws IOException;
   private static native void nativeDestroy(long h);
 
   /** DataOutputStream target that appends to the direct batch buffer. */

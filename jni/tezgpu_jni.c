@@ -82,6 +82,20 @@ JNIEXPORT void JNICALL SORTER(nativeReset)(JNIEnv *env, jclass cls, jlong h) {
   failed(env, tezgpu_sorter_reset((tezgpu_sorter *)(intptr_t)h));
 }
 
+JNIEXPORT void JNICALL SORTER(nativeSetCombiner)(JNIEnv *env, jclass cls, jlong h, jint kind) {
+  (void)cls;
+  failed(env, tezgpu_sorter_set_combiner((tezgpu_sorter *)(intptr_t)h, kind));
+}
+
+JNIEXPORT void JNICALL SORTER(nativeCombineInfo)(JNIEnv *env, jclass cls, jlong h, jlongArray info) {
+  (void)cls;
+  uint64_t in = 0, out = 0;
+  if (!failed(env, tezgpu_sorter_combine_info((tezgpu_sorter *)(intptr_t)h, &in, &out, NULL))) {
+    jlong v[2] = {(jlong)in, (jlong)out};
+    (*env)->SetLongArrayRegion(env, info, 0, 2, v);
+  }
+}
+
 JNIEXPORT void JNICALL SORTER(nativeDestroy)(JNIEnv *env, jclass cls, jlong h) {
   (void)env; (void)cls;
   tezgpu_sorter_destroy((tezgpu_sorter *)(intptr_t)h);
@@ -126,6 +140,11 @@ JNIEXPORT void JNICALL MERGER(nativeSetCheckForSameKeys)(JNIEnv *env, jclass cls
   failed(env, tezgpu_merge_set_check_for_same_keys((tezgpu_merger *)(intptr_t)h, on ? 1 : 0));
 }
 
+JNIEXPORT void JNICALL MERGER(nativeSetCombiner)(JNIEnv *env, jclass cls, jlong h, jint kind) {
+  (void)cls;
+  failed(env, tezgpu_merge_set_combiner((tezgpu_merger *)(intptr_t)h, kind));
+}
+
 JNIEXPORT jint JNICALL MERGER(nativeNextBatch)(JNIEnv *env, jclass cls, jlong h, jobject out, jint cap, jobject idx, jint idx_cap) {
   (void)cls;
   uint32_t n = 0;
@@ -162,5 +181,6 @@ JNIEXPORT void JNICALL MERGER(nativeClose)(JNIEnv *env, jclass cls, jlong h) {
 /* nativeMergeSpills (PipelinedSorter.flush's final merge) reads the spill files and their TezSpillRecord indexes and
  * builds the partition-tagged segment table exactly as tez_b200/csrc/host/tez_runtime_library.cc::GpuSorter::flush does
  * (:281-330): tezgpu_merge_open(conf with num_partitions = P) -> tezgpu_merge_set_check_for_same_keys(needsRLE) ->
- * tezgpu_merge_write_partitions(out, index, rle = needsRLE).  It is that C++ code behind a JNI signature; kept there so
+ * tezgpu_merge_set_combiner(kind, when numSpills >= combine.min.spills) -> tezgpu_merge_write_partitions(out, index,
+ * rle = needsRLE).  It is that C++ code behind a JNI signature; kept there so
  * the logic exists once and is exercised by tests/test_runtime_library_gpu.py. */

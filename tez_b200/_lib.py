@@ -62,6 +62,8 @@ SYMBOLS = [
     ("tezgpu_sorter_reset", C.c_int32, [_V]),
     ("tezgpu_sorter_sort_device_fixed", C.c_int32, [_V, _V, _V, C.c_uint64, _V, C.c_uint64, _P(C.c_uint64), _V, _P(Stats)]),
     ("tezgpu_sorter_stream", _V, [_V]),
+    ("tezgpu_sorter_set_combiner", C.c_int32, [_V, C.c_int32]),
+    ("tezgpu_sorter_combine_info", C.c_int32, [_V, _P(C.c_uint64), _P(C.c_uint64), _P(C.c_float)]),
     ("tezgpu_shuffle_header_size", C.c_uint64, [C.c_char_p, C.c_int64, C.c_int64, C.c_int32]),
     ("tezgpu_shuffle_header_write", C.c_int32, [C.c_char_p, C.c_int64, C.c_int64, C.c_int32, _V, C.c_uint64, _P(C.c_uint64)]),
     ("tezgpu_shuffle_header_read", C.c_int32, [_V, C.c_uint64, _V, C.c_uint64, _P(C.c_int64), _P(C.c_int64), _P(C.c_int32), _P(C.c_uint64)]),
@@ -83,6 +85,8 @@ SYMBOLS = [
     ("tezgpu_merge_write_ifile_device", C.c_int32, [_V, _V, C.c_uint64, C.c_int32, _P(C.c_int64), _P(C.c_int64), _P(Stats)]),
     ("tezgpu_merge_write_partitions_device", C.c_int32, [_V, _V, C.c_uint64, C.c_int32, _P(C.c_uint64), _V, _P(Stats)]),
     ("tezgpu_merge_write_partitions", C.c_int32, [_V, C.c_char_p, C.c_char_p, C.c_int32, _V, _P(Stats)]),
+    ("tezgpu_merge_set_combiner", C.c_int32, [_V, C.c_int32]),
+    ("tezgpu_merge_combine_info", C.c_int32, [_V, _P(C.c_uint64), _P(C.c_uint64), _P(C.c_float)]),
     ("tezgpu_merge_stream", _V, [_V]),
     ("tezgpu_peer_alloc", C.c_int32, [C.c_int32, C.c_uint64, _P(_V), _V]),
     ("tezgpu_peer_free", C.c_int32, [C.c_int32, _V]),

@@ -66,6 +66,9 @@ static const char *K_FINAL_MERGE = "tez.runtime.enable.final-merge.in.output";  
 static const char *K_REPORT_STATS = "tez.runtime.report.partition.stats";       // :195-198 default memory_optimized
 static const char *K_COMPRESS = "tez.runtime.compress";
 static const char *K_SERIALIZATIONS = "io.serializations";
+static const char *K_VALUE_CLASS = "tez.runtime.value.class";
+static const char *K_COMBINER = "tez.runtime.combiner.class";
+static const char *K_COMBINE_MIN_SPILLS = "tez.runtime.combine.min.spills";  // :128-130 default 3
 
 static bool ends_with(const std::string &s, const char *suf) {
   size_t n = strlen(suf);
@@ -83,6 +86,30 @@ static int comparator_for(const Configuration &c) {
     return TEZGPU_CMP_BYTESWRITABLE;
   }
   throw Err(TEZGPU_E_UNSUPPORTED, "key class '" + key + "' has no device comparator (supported: Text, BytesWritable, IntWritable, LongWritable)");
+}
+
+// MRCombiner over a sum reducer runs on the device (TEZGPU_COMBINE_*).  MRCombiner takes the reducer class from
+// mapreduce.job.combine.class under the new API and from mapred.combiner.class otherwise (ConfigUtils.useNewApi,
+// RL/common/ConfigUtils.java:128-130).  Any other combiner class is not run, as before the device combiner existed.
+static int combiner_for(const Configuration &c) {
+  if (c.get(K_COMBINER, "") != "org.apache.tez.mapreduce.combine.MRCombiner") return TEZGPU_COMBINE_NONE;
+  const bool new_api = c.getBoolean("mapred.mapper.new-api", false);
+  const std::string red = c.get(new_api ? "mapreduce.job.combine.class" : "mapred.combiner.class", "");
+  int kind;
+  std::string need;
+  if (red == "org.apache.hadoop.mapreduce.lib.reduce.IntSumReducer") {
+    kind = TEZGPU_COMBINE_INT_SUM;
+    need = "org.apache.hadoop.io.IntWritable";
+  } else if (red == "org.apache.hadoop.mapreduce.lib.reduce.LongSumReducer" || red == "org.apache.hadoop.mapred.lib.LongSumReducer") {
+    kind = TEZGPU_COMBINE_LONG_SUM;
+    need = "org.apache.hadoop.io.LongWritable";
+  } else {
+    return TEZGPU_COMBINE_NONE;
+  }
+  // the reference would fail later, at the first spill, with a ClassCastException inside the reducer
+  const std::string val = c.get(K_VALUE_CLASS, "");
+  RT_CHECK(val == need, TEZGPU_E_UNSUPPORTED, "combiner " + red + " sums " + need + " values, but the value class is '" + val + "'");
+  return kind;
 }
 
 // ---------------------------------------------------------------- small utilities
@@ -191,11 +218,21 @@ struct GpuSorter {
   std::vector<int64_t> final_idx;
   std::vector<int64_t> partition_stats;  // partitionStats[p] += rawLength at every spill (SORT/PipelinedSorter.java:631-633)
   int last_spill_rle = 0;                // merger.needsRLE() of the most recent spill's SpanMerger (:599,805,814)
+  int combine_kind = TEZGPU_COMBINE_NONE;
+  long min_spills_for_combine = 3;
   std::map<std::string, int64_t> &counters;
 
-  GpuSorter(const tezgpu_conf &c, int64_t mem, bool fm, const std::string &wd, const std::string &u, std::map<std::string, int64_t> &ctr)
-      : gc(c), P(c.num_partitions), available_memory(mem), final_merge(fm), work_dir(wd), uid(u), counters(ctr) {
+  GpuSorter(const tezgpu_conf &c, int64_t mem, bool fm, const std::string &wd, const std::string &u, std::map<std::string, int64_t> &ctr,
+            int combiner, long min_spills)
+      : gc(c), P(c.num_partitions), available_memory(mem), final_merge(fm), work_dir(wd), uid(u), combine_kind(combiner),
+        min_spills_for_combine(min_spills), counters(ctr) {
     gpu_check(tezgpu_sorter_create(&gc, &h));
+    if (combine_kind != TEZGPU_COMBINE_NONE) gpu_check(tezgpu_sorter_set_combiner(h, combine_kind));
+  }
+  // TaskCounter.COMBINE_INPUT_RECORDS / COMBINE_OUTPUT_RECORDS of one combine (ValuesIterator / the combiner's writer)
+  void count_combine(uint64_t in, uint64_t out) {
+    counters["COMBINE_INPUT_RECORDS"] += (int64_t)in;
+    counters["COMBINE_OUTPUT_RECORDS"] += (int64_t)out;
   }
   ~GpuSorter() { if (h) tezgpu_sorter_destroy(h); }
 
@@ -241,6 +278,11 @@ struct GpuSorter {
     std::vector<int64_t> idx((size_t)P * 3);
     tezgpu_stats st;
     gpu_check(tezgpu_sorter_flush(h, f.c_str(), fi.c_str(), idx.data(), &st));
+    if (combine_kind != TEZGPU_COMBINE_NONE) {  // runCombineProcessor per partition at every spill (:601-609)
+      uint64_t in = 0, out = 0;
+      gpu_check(tezgpu_sorter_combine_info(h, &in, &out, nullptr));
+      count_combine(in, out);
+    }
     gpu_check(tezgpu_sorter_reset(h));
     // adjustSpillCounters (:468-482)
     if (!final_merge) counters["OUTPUT_BYTES_WITH_OVERHEAD"] += st.output_bytes_with_overhead;
@@ -311,10 +353,16 @@ struct GpuSorter {
     // TezMerger.merge(..., checkForSameKeys = merger.needsRLE()) into Writer(..., rle = merger.needsRLE()), `merger`
     // being the SpanMerger of the last spill (SORT/PipelinedSorter.java:797-814)
     int32_t rc = tezgpu_merge_set_check_for_same_keys(m, last_spill_rle);
+    // the combiner runs in the final merge once numSpills >= tez.runtime.combine.min.spills (:815-820)
+    const bool combine = combine_kind != TEZGPU_COMBINE_NONE && num_spills >= min_spills_for_combine;
+    if (rc == 0 && combine) rc = tezgpu_merge_set_combiner(m, combine_kind);
     if (rc == 0)
       rc = tezgpu_merge_write_partitions(m, final_out.c_str(), final_index.c_str(), /*rle=*/last_spill_rle, final_idx.data(), &st);
+    uint64_t cin = 0, cout = 0;
+    if (rc == 0 && combine) rc = tezgpu_merge_combine_info(m, &cin, &cout, nullptr);
     tezgpu_merge_close(m);
     gpu_check(rc);
+    if (combine) count_combine(cin, cout);
     const uint64_t len = (uint64_t)st.file_out_bytes;
     counters["SPILLED_RECORDS"] += st.spilled_records;
     int64_t raw = 0;
@@ -366,6 +414,8 @@ struct Output {
     RT_CHECK(sc == "PIPELINED" || sc == "LEGACY", TEZGPU_E_INVALID,
              "Invalid sorter class specified in config, propertyName=" + std::string(K_SORTER_CLASS) + ", value=" + sc + ", validValues=[LEGACY, PIPELINED]");
     RT_CHECK(!conf.getBoolean(K_COMPRESS, false), TEZGPU_E_UNSUPPORTED, "tez.runtime.compress=true: IFile codecs are not supported on the device path yet");
+    const int combiner = combiner_for(conf);
+    const long min_spills = conf.getInt(K_COMBINE_MIN_SPILLS, 3);
     tezgpu_conf gc;
     memset(&gc, 0, sizeof(gc));
     gc.abi_version = TEZGPU_ABI_VERSION;
@@ -378,7 +428,7 @@ struct Output {
     gc.send_empty_partition_details = send_empty ? 1 : 0;
     gc.sorter_impl = sc == "LEGACY" ? 1 : 0;
     gc.mem_budget_bytes = (uint64_t)granted;
-    sorter = new GpuSorter(gc, granted > 0 ? granted : requested, final_merge, work_dir, uid, counters);
+    sorter = new GpuSorter(gc, granted > 0 ? granted : requested, final_merge, work_dir, uid, counters, combiner, min_spills);
     started = true;
   }
   void write(const uint8_t *k, uint32_t kl, const uint8_t *v, uint32_t vl, int32_t partition) {

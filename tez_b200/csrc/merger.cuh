@@ -785,7 +785,7 @@ class Merger {
     int64_t index[3] = {0, 0, 0};
     uint64_t len = 0;
     tezgpu_stats st;
-    pipe.emit_phase(writer_rle ? 1 : 0, true, d_out_buf, cap, &len, index, &st);
+    pipe.emit_output(writer_rle ? 1 : 0, true, d_out_buf, cap, &len, index, &st);
     st.output_bytes = (int64_t)kv_bytes;
     st.kernel_launches += launches - pipe.state.launches;
     if (raw_len) *raw_len = index[1];
@@ -796,7 +796,7 @@ class Merger {
   void write_partitions_device(uint8_t *d_out_buf, uint64_t cap, int writer_rle, uint64_t *out_len, int64_t *index,
                                tezgpu_stats *stats) {
     tezgpu_stats st;
-    pipe.emit_phase(writer_rle ? 1 : 0, true, d_out_buf, cap, out_len, index, &st);
+    pipe.emit_output(writer_rle ? 1 : 0, true, d_out_buf, cap, out_len, index, &st);
     st.output_bytes = (int64_t)kv_bytes;
     st.kernel_launches += launches - pipe.state.launches;
     if (stats) *stats = st;

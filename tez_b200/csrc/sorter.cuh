@@ -15,6 +15,7 @@
 #include "emit_tma.cuh"
 #include "emit_runs.cuh"
 #include "sorter_kernels.cuh"
+#include "combine.cuh"
 
 namespace tezgpu {
 
@@ -136,6 +137,7 @@ class SortPipeline {
     int launches = 0;
     bool have_bounds = false, spec_layout = false;  // partition bounds / fixed-width layout already on the device
     uint64_t spec_file_bytes = 0, spec_tiles = 0;
+    const uint8_t *same = nullptr;  // equal-key flags when they are not the pipeline's own `same` (combined records)
   } state;
   // merge mode only (the Merger sets them): MergeQueue.checkForSameKeys, and "no input record was run-length encoded"
   // (every segment had the plain fixed framing), which together decide whether any record can be written as a repeat
@@ -153,7 +155,7 @@ class SortPipeline {
     memset(&e, 0, sizeof(e));
     e.rec = rec;
     e.order = order;
-    e.same = same.as<uint8_t>();
+    e.same = state.same ? state.same : same.as<uint8_t>();
     e.part_start = part_start.as<uint32_t>();
     e.seg_start = seg_start.as<uint64_t>();
     e.tile_start = tile_start.as<uint32_t>();
@@ -220,7 +222,175 @@ class SortPipeline {
     else if (conf.rle_policy == TEZGPU_RLE_OFF) rle = 0;
     else rle = (conf.sorter_impl == 1) ? 0 : ((double)state.dup_count > 0.1 * (double)rec.n);
     if (conf.sorter_impl == TEZGPU_SORTER_UNORDERED) rle = 0;   // Writer(..., codec, null, null): no run-length encoding (:1092)
-    emit_phase(rle, false, d_out, out_cap, out_len, index, stats);
+    emit_output(rle, false, d_out, out_cap, out_len, index, stats);
+  }
+
+  // ---------------- combiner (combine.cuh): TEZGPU_COMBINE_* of the handle; results of the last emit_output
+  int combine_kind = TEZGPU_COMBINE_NONE;
+  uint64_t combine_in = 0, combine_out = 0;
+  float combine_ms = 0;
+  DeviceBuffer c_vals, c_aggf, c_aggs, c_heads, c_carry, c_bad, c_idx, c_K, c_sum, c_order, c_same, c_sizes, c_koff, c_klen,
+      c_vlen, c_kv;
+  EventTimer c_timer;
+
+  // emit_phase of the sorted records, through the combiner when one is set.  The record view of the sort phase is
+  // restored afterwards, so the merger's record iterator still walks the uncombined stream.
+  void emit_output(int rle, bool merge_mode, uint8_t *d_out, uint64_t out_cap, uint64_t *out_len, int64_t *index,
+                   tezgpu_stats *stats) {
+    combine_in = combine_out = 0;
+    combine_ms = 0;
+    if (combine_kind == TEZGPU_COMBINE_NONE) {
+      emit_phase(rle, merge_mode, d_out, out_cap, out_len, index, stats);
+      return;
+    }
+    const SortState raw = state;
+    const bool combined = combine_phase();
+    try {
+      emit_phase(rle, merge_mode, d_out, out_cap, out_len, index, stats);
+    } catch (...) {
+      if (combined) { state = raw; state.have_bounds = state.spec_layout = false; }
+      throw;
+    }
+    if (combined) {
+      state = raw;
+      state.have_bounds = state.spec_layout = false;  // the emit overwrote the partition bounds and the layout
+    }
+    if (stats) {
+      // OUTPUT_RECORDS and the RLE inputs are counted before the combine, SPILLED_RECORDS / rawLength after it
+      stats->output_records = raw.rec.n;
+      stats->adjacent_equal_keys = (int64_t)raw.dup_count;
+      stats->tie_records = (int64_t)raw.tie_records;
+    }
+  }
+
+  // Replaces `state` by the combined records (one per group of equal keys, sorted, no two keys equal) and returns true;
+  // returns false when the sorted records already are their own combination (no two adjacent keys equal: the sum of one
+  // value is that value's bytes).  Value widths are checked either way.
+  bool combine_phase() {
+    const Records rec = state.rec;
+    const uint32_t n = rec.n;
+    const uint32_t vw = combine_kind == TEZGPU_COMBINE_INT_SUM ? 4u : 8u;
+    const char *what = vw == 4 ? " is not a 4-byte IntWritable" : " is not an 8-byte LongWritable";
+    combine_in = combine_out = n;
+    if (n == 0) return false;
+    if (rec.fixed) TG_CHECK(rec.vlen == vw, TEZGPU_E_INVALID, std::string("combiner value of record 0") + what);
+    if (state.dup_count == 0 && rec.fixed) return false;
+    c_timer.reset();
+    c_timer.mark(stream);
+    c_bad.ensure(16);
+    TG_CUDA(cudaMemsetAsync(c_bad.p, 0xFF, 4, stream));
+    uint32_t *bad = c_bad.as<uint32_t>();
+    uint64_t *hs = h_small.as<uint64_t>() + 48;
+    auto check_widths = [&]() {
+      TG_CUDA(cudaMemcpyAsync(&hs[2], bad, 4, cudaMemcpyDeviceToHost, stream));
+      TG_CUDA(cudaStreamSynchronize(stream));
+      const uint32_t b = (uint32_t)hs[2];
+      TG_CHECK(b == 0xFFFFFFFFu, TEZGPU_E_INVALID, "combiner value of record " + std::to_string(b) + what);
+    };
+    if (state.dup_count == 0) {
+      k_comb_check_widths<<<(uint32_t)div_up(n, 256), 256, 0, stream>>>(rec.val_len, n, vw, bad);
+      TG_CUDA(cudaGetLastError());
+      check_widths();
+      c_timer.mark(stream);
+      TG_CUDA(cudaStreamSynchronize(stream));
+      combine_ms = c_timer.ms(0, 1);
+      return false;
+    }
+    int launches = state.launches;
+    CombineParams cp;
+    cp.rec = rec;
+    cp.order = state.order;
+    cp.same = same.as<uint8_t>();
+    cp.n = n;
+    cp.vw = vw;
+    const uint32_t nblk = (uint32_t)div_up(n, SCAN_TILE);
+    c_vals.ensure((size_t)n * 8);
+    c_aggf.ensure((size_t)nblk * 4);
+    c_aggs.ensure((size_t)nblk * 8);
+    c_heads.ensure(((size_t)nblk + 2) * 8);
+    c_carry.ensure((size_t)nblk * 8);
+    // ---- segmented sum: reduce, scan the tile aggregates and head counts, apply
+    k_comb_reduce<<<nblk, SCAN_THREADS, 0, stream>>>(cp, c_vals.as<uint64_t>(), c_aggf.as<uint32_t>(), c_aggs.as<uint64_t>(),
+                                                     c_heads.as<uint64_t>(), bad);
+    k_scan_block_sums<<<1, 1024, 0, stream>>>(c_heads.as<uint64_t>(), nblk);
+    k_comb_carry<<<1, 1024, 0, stream>>>(c_aggf.as<uint32_t>(), c_aggs.as<uint64_t>(), nblk, c_carry.as<uint64_t>());
+    launches += 3;
+    TG_CUDA(cudaGetLastError());
+    TG_CUDA(cudaMemcpyAsync(&hs[0], c_heads.as<uint64_t>() + nblk, 8, cudaMemcpyDeviceToHost, stream));
+    check_widths();
+    const uint32_t m = (uint32_t)hs[0];
+    c_idx.ensure((size_t)m * 4);
+    c_K.ensure((size_t)m * 4);
+    c_sum.ensure((size_t)m * 8);
+    k_comb_apply<<<nblk, SCAN_THREADS, 0, stream>>>(cp, state.K, c_vals.as<uint64_t>(), c_heads.as<uint64_t>(),
+                                                    c_carry.as<uint64_t>(), c_idx.as<uint32_t>(), c_K.as<uint32_t>(),
+                                                    c_sum.as<uint64_t>());
+    launches++;
+    // ---- pack the m groups as records in sorted order
+    Records cr;
+    memset(&cr, 0, sizeof(cr));
+    cr.n = m;
+    cr.cmp = rec.cmp;
+    cr.hash_partition = rec.hash_partition;
+    cr.num_partitions = rec.num_partitions;
+    cr.pbits = rec.pbits;
+    const uint32_t g256 = (uint32_t)div_up(m, 256);
+    if (rec.fixed) {
+      const uint64_t bytes = (uint64_t)m * (rec.klen + vw);
+      c_kv.ensure(bytes + 32);
+      k_comb_pack<true><<<g256, 256, 0, stream>>>(rec, c_idx.as<uint32_t>(), c_sum.as<uint64_t>(), m, vw, nullptr,
+                                                  c_kv.as<uint8_t>(), nullptr, nullptr);
+      launches++;
+      cr.fixed = 1;
+      cr.klen = rec.klen;
+      cr.vlen = vw;
+      cr.kv_bytes = bytes;
+    } else {
+      const uint32_t mblk = (uint32_t)div_up(m, SCAN_TILE);
+      c_sizes.ensure((size_t)m * 4);
+      c_koff.ensure(((size_t)m + 2) * 8);
+      c_klen.ensure((size_t)m * 4);
+      c_vlen.ensure((size_t)m * 4);
+      blk.ensure(((size_t)mblk + 2) * 8);
+      k_comb_sizes<<<g256, 256, 0, stream>>>(rec, c_idx.as<uint32_t>(), m, vw, c_sizes.as<uint32_t>());
+      k_sum_u32_blocks<<<mblk, SCAN_THREADS, 0, stream>>>(c_sizes.as<uint32_t>(), m, blk.as<uint64_t>());
+      k_scan_block_sums<<<1, 1024, 0, stream>>>(blk.as<uint64_t>(), mblk);
+      k_scan_u32_apply<<<mblk, SCAN_THREADS, 0, stream>>>(c_sizes.as<uint32_t>(), m, blk.as<uint64_t>(), c_koff.as<uint64_t>());
+      launches += 4;
+      TG_CUDA(cudaGetLastError());
+      TG_CUDA(cudaMemcpyAsync(&hs[1], c_koff.as<uint64_t>() + m, 8, cudaMemcpyDeviceToHost, stream));
+      TG_CUDA(cudaStreamSynchronize(stream));
+      const uint64_t bytes = hs[1];
+      c_kv.ensure(align_up(bytes, 16) + 32);
+      k_comb_pack<false><<<g256, 256, 0, stream>>>(rec, c_idx.as<uint32_t>(), c_sum.as<uint64_t>(), m, vw, c_koff.as<uint64_t>(),
+                                                   c_kv.as<uint8_t>(), c_klen.as<uint32_t>(), c_vlen.as<uint32_t>());
+      launches++;
+      cr.key_off = c_koff.as<uint64_t>();
+      cr.key_len = c_klen.as<uint32_t>();
+      cr.val_len = c_vlen.as<uint32_t>();
+      cr.kv_bytes = align_up(bytes, 16);
+    }
+    cr.kv = c_kv.as<uint8_t>();
+    // identity order, no equal neighbours
+    c_order.ensure((size_t)m * 4);
+    c_same.ensure(m);
+    k_comb_iota<<<g256, 256, 0, stream>>>(c_order.as<uint32_t>(), m);
+    TG_CUDA(cudaMemsetAsync(c_same.p, 0, m, stream));
+    launches++;
+    TG_CUDA(cudaGetLastError());
+    c_timer.mark(stream);
+    TG_CUDA(cudaStreamSynchronize(stream));
+    combine_ms = c_timer.ms(0, 1);
+    combine_out = m;
+    state.rec = cr;
+    state.K = c_K.as<uint32_t>();
+    state.order = c_order.as<uint32_t>();
+    state.same = c_same.as<uint8_t>();
+    state.dup_count = 0;
+    state.launches = launches;
+    // the partition bounds and the speculative layout of the sort phase describe n records, not m
+    state.have_bounds = state.spec_layout = false;
+    return true;
   }
 
   // partition + sort: stage, radix sort of (sort word, index), tie refinement.  Leaves K / order / same / counts.
@@ -469,6 +639,7 @@ class SortPipeline {
     }
     timer.mark(stream);
     state.rec = rec;
+    state.same = nullptr;
     state.K = K;
     state.order = order;
     state.dup_count = dup_count;

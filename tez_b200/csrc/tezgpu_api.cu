@@ -331,6 +331,30 @@ int32_t tezgpu_sorter_sort_device_fixed(tezgpu_sorter *h, const void *d_kv, cons
 
 void *tezgpu_sorter_stream(tezgpu_sorter *h) { return h ? (void *)h->pipe.stream : nullptr; }
 
+int32_t tezgpu_sorter_set_combiner(tezgpu_sorter *h, int32_t kind) {
+  TG_API_BEGIN
+  TG_CHECK(h, TEZGPU_E_INVALID, "null handle");
+  TG_CHECK(kind >= TEZGPU_COMBINE_NONE && kind <= TEZGPU_COMBINE_LONG_SUM, TEZGPU_E_INVALID, "unknown combiner kind");
+  TG_CHECK(h->n == 0 && !h->flushed, TEZGPU_E_STATE, "set the combiner before the first collect or right after a reset");
+  TG_CHECK(kind == TEZGPU_COMBINE_NONE || h->pipe.conf.sorter_impl != TEZGPU_SORTER_UNORDERED, TEZGPU_E_UNSUPPORTED,
+           "an unordered output has no combiner (its records are not grouped by key)");
+  const uint32_t vw = kind == TEZGPU_COMBINE_INT_SUM ? 4 : 8;
+  TG_CHECK(kind == TEZGPU_COMBINE_NONE || h->pipe.conf.fixed_val_len == 0 || h->pipe.conf.fixed_val_len == vw, TEZGPU_E_INVALID,
+           "fixed_val_len " + std::to_string(h->pipe.conf.fixed_val_len) + " is not the combiner's value width (" +
+               std::to_string(vw) + " bytes)");
+  h->pipe.combine_kind = kind;
+  TG_API_END
+}
+
+int32_t tezgpu_sorter_combine_info(tezgpu_sorter *h, uint64_t *records_in, uint64_t *records_out, float *ms) {
+  TG_API_BEGIN
+  TG_CHECK(h, TEZGPU_E_INVALID, "null handle");
+  if (records_in) *records_in = h->pipe.combine_in;
+  if (records_out) *records_out = h->pipe.combine_out;
+  if (ms) *ms = h->pipe.combine_ms;
+  TG_API_END
+}
+
 // ------------------------------------------------------------------------------------------------ NVLink peer fetch
 int32_t tezgpu_peer_alloc(int32_t device, uint64_t bytes, void **dptr, uint8_t *handle_out) {
   TG_API_BEGIN

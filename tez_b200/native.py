@@ -32,13 +32,30 @@ def make_conf(num_partitions, comparator=CMP_BYTES, partitioner=PART_HASH, rle_p
     return c
 
 
+def _combine_info(fn, h):
+    i, o, ms = C.c_uint64(), C.c_uint64(), C.c_float()
+    check(fn(h, C.byref(i), C.byref(o), C.byref(ms)))
+    return i.value, o.value, ms.value
+
+
 class GpuSorter:
-    def __init__(self, num_partitions, **kw):
+    def __init__(self, num_partitions, combiner=COMBINE_NONE, **kw):
         self.L = _lib.load()
         self.conf = make_conf(num_partitions, **kw)
         self.P = num_partitions
         self.h = C.c_void_p()
         check(self.L.tezgpu_sorter_create(C.byref(self.conf), C.byref(self.h)))
+        if combiner != COMBINE_NONE:
+            self.set_combiner(combiner)
+
+    def set_combiner(self, kind):
+        """COMBINE_INT_SUM / COMBINE_LONG_SUM: every flush writes one record per group of equal keys with the summed
+        value (MRCombiner + IntSumReducer / LongSumReducer).  Before the first collect or right after reset()."""
+        check(self.L.tezgpu_sorter_set_combiner(self.h, kind))
+
+    def combine_info(self):
+        """(records into, records out of, device ms of) the combine of the last flush."""
+        return _combine_info(self.L.tezgpu_sorter_combine_info, self.h)
 
     def close(self):
         if self.h:
@@ -177,6 +194,14 @@ class GpuMerger:
     def set_check_for_same_keys(self, on):
         """MergeQueue's checkForSameKeys (SORT/TezMerger.java:560-573); default True."""
         check(self.L.tezgpu_merge_set_check_for_same_keys(self.h, 1 if on else 0))
+
+    def set_combiner(self, kind):
+        """Combiner of the write_* calls (a combining final merge); records() stays the uncombined stream."""
+        check(self.L.tezgpu_merge_set_combiner(self.h, kind))
+
+    def combine_info(self):
+        """(records into, records out of, device ms of) the combine of the last write."""
+        return _combine_info(self.L.tezgpu_merge_combine_info, self.h)
 
     def parse_info(self):
         """(mode, windows walked by hand) of the last open: 0 records addressed in place, 1 window parser, 2 sequential walker."""
