@@ -17,6 +17,11 @@ constexpr int FE_THREADS = 256;
 constexpr int FE_MAX_RECS = 256;
 constexpr int FE_IMG_BYTES = 22016;  // 256 records * 82 B + lead + header + EOF, multiple of 16
 
+// the source-oriented kernels build a whole tile in one FE_IMG_BYTES image: at least one record plus the worst-case
+// lead (15), segment header (4) and EOF markers (2) must fit.  Larger records take the general kernel (k_emit<true>),
+// which splits a tile over several images.
+static inline bool fast_emit_fits(uint32_t rec_size) { return (uint64_t)rec_size + 15 + 4 + 2 <= (uint64_t)FE_IMG_BYTES; }
+
 struct TileDesc {
   uint32_t p;      // partition
   uint32_t r0;     // first sorted position

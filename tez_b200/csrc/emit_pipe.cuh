@@ -26,13 +26,14 @@ namespace tezgpu {
 constexpr int FE4_BATCH = FE_THREADS / 32;  // one parked tile per warp
 constexpr int FE4_UNROLL = TEZGPU_EMIT4_MAP16 ? 6 : 5;  // gather rounds held in registers
 
-// can a tile of `recs` records with `cpr` pieces each be gathered in FE4_UNROLL rounds?
+// can a tile of `recs` records with `cpr` pieces each be gathered in FE4_UNROLL rounds?  Both maps need cpr <= 8: the
+// packed piece map of full tiles (k_emit_fast4) keeps 16c in a 7-bit field, so piece 8 and up would alias piece c % 8.
 static inline bool emit4_fits(uint32_t recs, uint32_t cpr) {
 #if TEZGPU_EMIT4_MAP16
   const uint32_t rph = 16u / cpr;
   return cpr <= 8 && 16ull * ((recs + rph - 1) / rph) <= (uint64_t)FE4_UNROLL * FE_THREADS;
 #else
-  return (uint64_t)recs * cpr <= (uint64_t)FE4_UNROLL * FE_THREADS;
+  return cpr <= 8 && (uint64_t)recs * cpr <= (uint64_t)FE4_UNROLL * FE_THREADS;
 #endif
 }
 
@@ -136,8 +137,9 @@ __global__ void __launch_bounds__(FE_THREADS * SUBS, SUBS > 1 ? 1 : TEZGPU_EMIT4
   };
 #endif
   // Full tiles (all but the last of a partition) share one piece map: packed once per thread as
-  // j | 16c << 8 | (j * rec_size + hdr_len + 16c) << 15, so a piece costs an index look-up and one multiply-add
-  // instead of the divide / permute arithmetic (which was ~25 % of the kernel's instructions).
+  // j | 16c << 8 | (j * rec_size + hdr_len + 16c) << 15 (16c < 128: emit4_fits admits cpr <= 8 only), so a piece
+  // costs an index look-up and one multiply-add instead of the divide / permute arithmetic (which was ~25 % of the
+  // kernel's instructions).
   const uint32_t full_nr = e.recs_per_tile;
   uint32_t pk[UNROLL], onmask = 0;
 #pragma unroll

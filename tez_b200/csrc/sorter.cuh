@@ -181,7 +181,8 @@ class SortPipeline {
     for (int b = 0; b < vint_size_u32(rec.vlen); b++) e.fixed_hdr[h++] = vint_byte_u32(rec.vlen, b);
     e.fixed_hdr_len = h;
     e.rec_size = h + rec.klen + rec.vlen;
-    // the tile image must fit the image buffer of the source-oriented emit kernels (FE_IMG_BYTES)
+    // the tile image must fit the image buffer of the source-oriented emit kernels (FE_IMG_BYTES); a record that does
+    // not fit it alone (!fast_emit_fits) gets one-record tiles, which the general kernel splits over several images
     e.recs_per_tile = std::max<uint32_t>(1, std::min<uint32_t>(EMIT_MAX_RECS, (FE_IMG_BYTES - 32) / e.rec_size));
     // Round filling: the checksum / write-out loop of the source-oriented kernels walks a tile in rounds of
     // FE_THREADS 16-byte chunks; 256 records of 82 bytes are 5.13 rounds, six are executed.  Among the tile sizes
@@ -721,7 +722,8 @@ class SortPipeline {
     // fixed-width records take the source-oriented kernel (emit_fast.cuh): 16-byte aligned packed records use one
     // 128-bit load per piece, records at explicit / unaligned offsets two loads + a funnel shift
     const uint32_t stride = rec.klen + rec.vlen;
-    const bool fast_emit = fixed_emit && stride >= 16 && (stride % 16 == 0) && !getenv("TEZGPU_NO_FAST_EMIT");
+    const bool fast_emit = fixed_emit && stride >= 16 && (stride % 16 == 0) && fast_emit_fits(e.rec_size) &&
+                           !getenv("TEZGPU_NO_FAST_EMIT");
     const bool fast_aligned = fast_emit && !rec.key_off && !rec.use_runs && (((uintptr_t)rec.kv & 15u) == 0);
     FastEmitParams fp;
     if (tiles && fast_emit) {
