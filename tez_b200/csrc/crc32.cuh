@@ -143,8 +143,9 @@ struct WarpLinearMap {
 // x^(128*(T-1)) this adds to every partial is divided out once, in the per-lane alignment multiplier of the final fold
 // (CrcTables::einv; the inverse exists because the CRC-32 polynomial is primitive: tests/test_abi_cpu.py).
 // The third digit table costs 7 registers: measured on B200, kernels already at their register cap lose more to the
-// spills than they gain (k_emit_fast4 at 80 registers: 5.44 -> 6.94 ms, k_emit_fast4u 8.5 -> 9.8 ms), kernels with
-// headroom gain a little (k_emit_runs 8.98 -> 8.85 ms).  Hence a template flag per kernel.
+// spills than they gain (k_emit_fast4 with its gather in registers, at 80: 5.44 -> 6.94 ms, k_emit_fast4u 8.5 -> 9.8 ms),
+// kernels with headroom gain a little (k_emit_runs 8.98 -> 8.85 ms) or nothing (k_emit_fast4 with its gather in shared
+// memory: 4.99 ms either way).  Hence a template flag per kernel.
 template <bool ILP>
 struct CrcChunkFoldT {
   WarpLinearMap w, s;

@@ -5,10 +5,10 @@
 // 25 % of the warp samples waiting on the gather's global loads, 19 % at barriers (11 % of it behind warp 0 folding
 // the tile's partial checksums while seven warps idle).  This kernel keeps the same tile algorithm and byte-exact
 // output but reorders the work of a persistent CTA:
-//   * the 128-bit gather loads of tile N+1 are issued into registers BEFORE the checksum / write-out loop of tile N
-//     and stored to the image after it (record indices are fetched two tiles ahead, tile descriptors three), so the
-//     DRAM latency of the random gather hides behind ~190 instructions per thread-chunk of CRC work;
-//   * the per-tile second-level checksum fold is deferred: partials of FE4_BATCH tiles are parked in shared memory
+//   * the gather of tiles N+1 .. N+D is in flight while tile N is imaged, checksummed and written.  In k_emit_fast4<.,1>
+//     each thread copies its pieces with cp.async (LDGSTS) into a thread-private ring of D stages in shared memory,
+//     so the bytes in flight hold no registers; record indices are fetched D+1 tiles ahead, descriptors D+2;
+//   * the per-tile second-level checksum fold is deferred: partials of a batch of tiles are parked in shared memory
 //     and folded together, one tile per warp, so no warp waits for another's serial fold;
 //   * two barriers per tile instead of three.
 #pragma once
@@ -20,11 +20,16 @@
 #ifndef TEZGPU_EMIT4_MAP16
 #define TEZGPU_EMIT4_MAP16 0
 #endif
+#ifndef TEZGPU_EMIT4_STAGES
+#define TEZGPU_EMIT4_STAGES 1  // depth of k_emit_fast4<.,1>'s cp.async ring (profiles/README.md, round 3: 2 and 3 gain nothing)
+#endif
 
 namespace tezgpu {
 
 constexpr int FE4_BATCH = FE_THREADS / 32;  // one parked tile per warp
-constexpr int FE4_UNROLL = TEZGPU_EMIT4_MAP16 ? 6 : 5;  // gather rounds held in registers
+constexpr int FE4_UNROLL = TEZGPU_EMIT4_MAP16 ? 6 : 5;  // gather rounds per tile
+constexpr size_t SM_SMEM_BYTES = 228 * 1024;   // shared memory per SM (sm_100) ...
+constexpr size_t SM_SMEM_PER_CTA = 1024;       // ... of which the runtime reserves this much per resident CTA
 
 // can a tile of `recs` records with `cpr` pieces each be gathered in FE4_UNROLL rounds?  Both maps need cpr <= 8: the
 // packed piece map of full tiles (k_emit_fast4) keeps 16c in a 7-bit field, so piece 8 and up would alias piece c % 8.
@@ -58,19 +63,47 @@ __device__ __forceinline__ uint4 lds_v4(uint32_t a) {
 //           Measured on the SHFL-only kernel: a SHFL occupies the LSU data pipe for two cycles, so its 28 SHFL per
 //           chunk cost as much pipe time as the conflicting byte-table look-ups they replaced; the pipe, not issue
 //           or DRAM, bounded the kernel.
+//           Its 219 KB of tables leave no room for a cp.async ring, so its pieces wait in registers (STAGES = 0, the
+//           loads of tile N+1 in flight during tile N).
+// Per group: image | ring [STAGES][UNROLL][FE_THREADS] x 16 B (piece u of thread t at [s][u][t]: conflict-free) |
+// descriptors of tiles N .. N+D+2 | parked fold metadata | record indices of tiles N+D, N+D+1 | parked partials.
+// BATCH (tiles parked per fold) is a warp's worth where TEZGPU_EMIT4_MIN_CTAS CTAs still fit an SM, half that otherwise.
 template <int SUBS>
 struct Emit4Smem {
-  static constexpr int BATCH = SUBS > 1 ? 4 : FE4_BATCH;
+  static constexpr int STAGES = SUBS > 1 ? 0 : TEZGPU_EMIT4_STAGES;
+  static constexpr int DEPTH = STAGES > 0 ? STAGES : 1;  // tiles whose gather is in flight
+  static constexpr int NIDX = DEPTH + 1, NDESC = DEPTH + 3;
   static constexpr size_t WTAB = SUBS > 1 ? (size_t)4 * 256 * 32 * 4 : 0;
   static constexpr size_t SHARED = WTAB + 256 * 4 + 4 * 256 * 4;
-  static constexpr size_t GROUP = FE_IMG_BYTES + 3 * FE_MAX_RECS * 4 + (size_t)BATCH * FE_THREADS * 4 + (size_t)BATCH * sizeof(FoldMeta);
+  static constexpr size_t RING = FE_IMG_BYTES;
+  static constexpr size_t DESC = RING + (size_t)STAGES * FE4_UNROLL * FE_THREADS * 16;
+  static constexpr size_t META = DESC + NDESC * sizeof(TileDesc);
+  static constexpr size_t group_bytes(int batch) {
+    return META + (size_t)batch * sizeof(FoldMeta) + NIDX * FE_MAX_RECS * 4 + (size_t)batch * FE_THREADS * 4;
+  }
+  static constexpr int BATCH =
+      SUBS > 1 ? 4 : TEZGPU_EMIT4_MIN_CTAS * (SHARED + group_bytes(FE4_BATCH) + SM_SMEM_PER_CTA) <= SM_SMEM_BYTES ? FE4_BATCH : FE4_BATCH / 2;
+  static constexpr size_t IDX = META + (size_t)BATCH * sizeof(FoldMeta);
+  static constexpr size_t PART = IDX + NIDX * FE_MAX_RECS * 4;
+  static constexpr size_t GROUP = group_bytes(BATCH);
   static constexpr size_t TOTAL = SHARED + SUBS * GROUP;
 };
+static_assert(TEZGPU_EMIT4_MIN_CTAS * (Emit4Smem<1>::TOTAL + SM_SMEM_PER_CTA) <= SM_SMEM_BYTES, "k_emit_fast4 ring does not fit its CTAs/SM");
+static_assert(Emit4Smem<3>::TOTAL + SM_SMEM_PER_CTA <= SM_SMEM_BYTES, "k_emit_fast4<.,3> does not fit an SM");
+
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void *src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 template <int UNROLL, int SUBS>
 __global__ void __launch_bounds__(FE_THREADS * SUBS, SUBS > 1 ? 1 : TEZGPU_EMIT4_MIN_CTAS) k_emit_fast4(FastEmitParams fp) {
   using L = Emit4Smem<SUBS>;
-  constexpr int BATCH = L::BATCH;
+  static_assert(UNROLL <= FE4_UNROLL, "ring stage sized for FE4_UNROLL pieces per thread");
+  constexpr int BATCH = L::BATCH, D = L::DEPTH;
+  constexpr bool RING = L::STAGES > 0;
   extern __shared__ __align__(16) uint8_t smem4[];
   uint32_t *s_wtab = reinterpret_cast<uint32_t *>(smem4);              // [4][256][32] lane-private (SUBS > 1)
   uint32_t *s_tab = reinterpret_cast<uint32_t *>(smem4 + L::WTAB);     // classic byte table (trailing bytes)
@@ -78,9 +111,12 @@ __global__ void __launch_bounds__(FE_THREADS * SUBS, SUBS > 1 ? 1 : TEZGPU_EMIT4
   const int sub = threadIdx.x / FE_THREADS, tid = threadIdx.x % FE_THREADS, lane = tid & 31, warp = tid >> 5;
   uint8_t *gbase = smem4 + L::SHARED + (size_t)sub * L::GROUP;
   uint8_t *s_img = gbase;
-  uint32_t(*s_idx)[FE_MAX_RECS] = reinterpret_cast<uint32_t(*)[FE_MAX_RECS]>(gbase + FE_IMG_BYTES);  // tiles N, N+1, N+2
-  uint32_t(*s_part)[FE_THREADS] = reinterpret_cast<uint32_t(*)[FE_THREADS]>(gbase + FE_IMG_BYTES + 3 * FE_MAX_RECS * 4);
-  FoldMeta *s_meta = reinterpret_cast<FoldMeta *>(gbase + FE_IMG_BYTES + 3 * FE_MAX_RECS * 4 + (size_t)BATCH * FE_THREADS * 4);
+  TileDesc *s_desc = reinterpret_cast<TileDesc *>(gbase + L::DESC);                                  // ring of NDESC tiles
+  FoldMeta *s_meta = reinterpret_cast<FoldMeta *>(gbase + L::META);
+  uint32_t(*s_idx)[FE_MAX_RECS] = reinterpret_cast<uint32_t(*)[FE_MAX_RECS]>(gbase + L::IDX);      // ring of NIDX tiles
+  uint32_t(*s_part)[FE_THREADS] = reinterpret_cast<uint32_t(*)[FE_THREADS]>(gbase + L::PART);
+  // this thread's slot of piece u in ring stage s: + (s * UNROLL + u) * FE_THREADS * 16
+  const uint32_t ring_base = (uint32_t)__cvta_generic_to_shared(gbase + L::RING) + 16u * tid;
   auto group_sync = [&]() {
     if (SUBS == 1) __syncthreads();
     else asm volatile("bar.sync %0, %1;" ::"r"(sub + 1), "r"(FE_THREADS) : "memory");
@@ -149,10 +185,11 @@ __global__ void __launch_bounds__(FE_THREADS * SUBS, SUBS > 1 ? 1 : TEZGPU_EMIT4
     pk[u] = on ? (j | (16u * c) << 8 | (j * rec_size + hdr_len + 16u * c) << 15) : 0u;
     onmask |= on ? 1u << u : 0u;
   }
-  uint4 v[UNROLL];
+  uint4 v[UNROLL];  // STAGES = 0: the pieces of the tile in flight
+  constexpr uint32_t STAGE_STRIDE = (uint32_t)UNROLL * FE_THREADS * 16;
   // all addresses first, then the loads back to back (keeps ptxas from reusing the destination registers of later
   // rounds as temporaries between the loads)
-  auto issue_gather = [&](uint32_t nr, const uint32_t *idx) {
+  auto issue_gather = [&](uint32_t nr, const uint32_t *idx, uint32_t stage) {
     const uint8_t *src[UNROLL];
     bool on[UNROLL];
     if (nr == full_nr) {
@@ -171,60 +208,76 @@ __global__ void __launch_bounds__(FE_THREADS * SUBS, SUBS > 1 ? 1 : TEZGPU_EMIT4
     }
     if (UNROLL == 5) asm volatile("" : "+l"(src[0]), "+l"(src[1]), "+l"(src[2]), "+l"(src[3]), "+l"(src[UNROLL - 1]));
 #pragma unroll
-    for (int u = 0; u < UNROLL; u++)
-      if (on[u]) v[u] = ldg_stream_v4(src[u]);
+    for (int u = 0; u < UNROLL; u++) {
+      if (!on[u]) continue;
+      if (RING) cp_async16(stage + u * FE_THREADS * 16, src[u]);
+      else v[u] = ldg_stream_v4(src[u]);
+    }
   };
+  auto landed = [&](int u, uint32_t stage) -> uint4 { return RING ? lds_v4(stage + u * FE_THREADS * 16) : v[u]; };
   // vint(klen) vint(vlen) of the fixed framing as one 16-bit store when it is two bytes at an even address
   const uint32_t hdr16 = (uint32_t)e.fixed_hdr[0] | (uint32_t)e.fixed_hdr[1] << 8;
 
-  // ---- prologue: descriptors of tiles 0..2 of this CTA, indices of tiles 0 and 1, gather of tile 0 in flight
-  uint32_t nr0, fl0, nr1 = 0, fl1 = 0, r0_2 = 0, nr2 = 0;
-  uint64_t abs0, abs1 = 0;
-  {
-    const TileDesc t0 = tiles[tile];
-    nr0 = t0.nr; fl0 = t0.flags; abs0 = t0.abs0;
-    if ((uint32_t)tid < nr0) s_idx[0][tid] = e.order[t0.r0 + tid];
-    if (tile + G < ntiles) {
-      const TileDesc t1 = tiles[tile + G];
-      nr1 = t1.nr; fl1 = t1.flags; abs1 = t1.abs0;
-      if ((uint32_t)tid < nr1) s_idx[1][tid] = e.order[t1.r0 + tid];
+  // ---- prologue: descriptors of tiles 0 .. D+1 of this group, indices of tiles 0 .. D, gathers of tiles 0 .. D-1
+  // in flight (one cp.async group per tile, also for tiles past the end, so that "tile N landed" is always
+  // wait_group D-1)
+  for (int k = 0; k < D + 2; k++) {
+    const uint64_t t = tile + (uint64_t)k * G;
+    if (t >= ntiles) break;
+    if (k <= D) {
+      const uint32_t r0 = tiles[t].r0, nrk = tiles[t].nr;
+      if ((uint32_t)tid < nrk) s_idx[k][tid] = e.order[r0 + tid];
     }
-    if (tile + 2 * (uint64_t)G < ntiles) { r0_2 = tiles[tile + 2 * G].r0; nr2 = tiles[tile + 2 * G].nr; }
+    if (tid < 8) reinterpret_cast<uint32_t *>(s_desc + k)[tid] = reinterpret_cast<const uint32_t *>(tiles + t)[tid];
   }
   group_sync();
-  issue_gather(nr0, s_idx[0]);
+#pragma unroll
+  for (int k = 0; k < D; k++) {
+    if (tile + (uint64_t)k * G < ntiles) issue_gather(s_desc[k].nr, s_idx[k], ring_base + k * STAGE_STRIDE);
+    if (RING) cp_async_commit();
+  }
 
-  uint32_t n_it = 0, slot = 0;
+  uint32_t n_it = 0, slot = 0, stage = ring_base;  // stage: ring stage of tile N (and of tile N+D)
   for (;; tile += G, n_it++) {
-    const bool has1 = tile + G < ntiles, has2 = tile + 2 * (uint64_t)G < ntiles, has3 = tile + 3 * (uint64_t)G < ntiles;
-    const uint32_t nr = nr0;
-    const bool first_tile = fl0 & 1u, last_tile = fl0 & 2u;
+    const bool has1 = tile + G < ntiles;
+    const bool hasD = tile + (uint64_t)D * G < ntiles, hasD1 = tile + (D + 1ull) * G < ntiles, hasD2 = tile + (D + 2ull) * G < ntiles;
+    const TileDesc &cur = s_desc[n_it % L::NDESC];
+    const uint32_t nr = cur.nr, fl = cur.flags;
+    const uint64_t abs0 = cur.abs0;
+    const bool first_tile = fl & 1u, last_tile = fl & 2u;
     const uint32_t lead = (uint32_t)(abs0 & 15u);
     const uint32_t rec0 = lead + (first_tile ? 4u : 0u);
     const uint32_t body_end = rec0 + nr * rec_size + (last_tile ? 2u : 0u);
 
-    // ---- prefetches that are consumed at the end of this iteration / in the next one
-    uint32_t r_idx = 0, r0_3 = 0, nr3 = 0, nr2n = 0, fl2n = 0;
-    uint64_t abs2n = 0;
-    if (has2) {
-      if ((uint32_t)tid < nr2) r_idx = e.order[r0_2 + tid];
-      const TileDesc *t2 = tiles + tile + 2 * (uint64_t)G;
-      nr2n = t2->nr; fl2n = t2->flags; abs2n = t2->abs0;
+    // ---- prefetches that are parked in shared memory at the end of this iteration: indices of tile N+D+1,
+    // descriptor of tile N+D+2 (one word per thread of the first eight)
+    uint32_t r_idx = 0, d_word = 0;
+    if (hasD1) {
+      const TileDesc &t1 = s_desc[(n_it + D + 1) % L::NDESC];
+      if ((uint32_t)tid < t1.nr) r_idx = e.order[t1.r0 + tid];
     }
-    if (has3) { const TileDesc *t3 = tiles + tile + 3 * (uint64_t)G; r0_3 = t3->r0; nr3 = t3->nr; }
+    if (hasD2 && tid < 8) d_word = reinterpret_cast<const uint32_t *>(tiles + tile + (D + 2ull) * G)[tid];
 
-    // ---- this tile's pieces (loaded during the previous iteration) -> image; framing
+    // ---- this tile's pieces (in flight since iteration N-D) -> image
+    if (RING) cp_async_wait<D - 1>();  // this thread's copies of tile N have landed (and are visible to it)
     if (nr == full_nr) {
 #pragma unroll
       for (int u = 0; u < UNROLL; u++)
-        if ((onmask >> u) & 1u) sts16_unaligned(img_base + rec0 + (pk[u] >> 15), v[u]);
+        if ((onmask >> u) & 1u) sts16_unaligned(img_base + rec0 + (pk[u] >> 15), landed(u, stage));
     } else {
 #pragma unroll
       for (int u = 0; u < UNROLL; u++) {
         uint32_t j, c;
-        if (piece(u, nr, j, c)) sts16_unaligned(img_base + rec0 + j * rec_size + hdr_len + 16u * c, v[u]);
+        if (piece(u, nr, j, c)) sts16_unaligned(img_base + rec0 + j * rec_size + hdr_len + 16u * c, landed(u, stage));
       }
     }
+    // ---- the gather of tile N+D reuses the stage (or registers) just read; it lands while tiles N .. N+D-1 are
+    // checksummed and written.  Every value read from the stage has been stored to the image above: the stores
+    // wait for the loads' data, and a thread issues in order, so the copies cannot overwrite a slot before its read.
+    if (hasD) issue_gather(s_desc[(n_it + D) % L::NDESC].nr, s_idx[(n_it + D) % L::NIDX], stage);
+    if (RING) cp_async_commit();
+    stage = (n_it + 1) % D == 0 ? ring_base : stage + STAGE_STRIDE;
+    // ---- framing
     if ((uint32_t)tid < nr) {
       const uint32_t a = img_base + rec0 + tid * rec_size;
       if (hdr_len == 2 && !(a & 1u)) sts_b16(a, hdr16);
@@ -235,9 +288,6 @@ __global__ void __launch_bounds__(FE_THREADS * SUBS, SUBS > 1 ? 1 : TEZGPU_EMIT4
       if (last_tile) { s_img[body_end - 2] = 0xFF; s_img[body_end - 1] = 0xFF; }
     }
     group_sync();  // (B) image complete
-
-    // ---- gather of the next tile goes out now; it lands while this tile is checksummed and written
-    if (has1) issue_gather(nr1, s_idx[(n_it + 1) % 3]);
 
     // ---- fused CRC + write-out (emit_fast.cuh): thread t owns the chunks at distance == T-1-t (mod T) from the end
     const uint32_t cb0 = rec0, cb1 = body_end;
@@ -296,9 +346,10 @@ __global__ void __launch_bounds__(FE_THREADS * SUBS, SUBS > 1 ? 1 : TEZGPU_EMIT4
       m.end = cb1 & 15u;
       s_meta[slot] = m;
     }
-    if (has2) s_idx[(n_it + 2) % 3][tid] = r_idx;
+    if (hasD1) s_idx[(n_it + D + 1) % L::NIDX][tid] = r_idx;
+    if (hasD2 && tid < 8) reinterpret_cast<uint32_t *>(s_desc + (n_it + D + 2) % L::NDESC)[tid] = d_word;
     slot++;
-    group_sync();  // (C) image free, partials / indices visible
+    group_sync();  // (C) image free, partials / indices / descriptor visible
 
     if (slot == (uint32_t)BATCH || !has1) {
       // ---- deferred second level: warp w folds parked tile w.  lane l folds partials l, l+32, ... (Horner with
@@ -333,13 +384,6 @@ __global__ void __launch_bounds__(FE_THREADS * SUBS, SUBS > 1 ? 1 : TEZGPU_EMIT4
       // the parked rows are rewritten only after barrier (B) of the next iteration, which every folding warp joins
     }
     if (!has1) break;
-    // the descriptor prefetches are consumed HERE: without this the compiler renames them straight into the next
-    // iteration, where their scoreboard is shared with the freshly issued gather loads and the first use stalls on
-    // those (measured: 20 % of all warp samples on one integer add in the middle of the gather)
-    asm volatile("" : "+r"(nr2n), "+r"(fl2n), "+l"(abs2n), "+r"(r0_3), "+r"(nr3));
-    nr0 = nr1; fl0 = fl1; abs0 = abs1;
-    nr1 = nr2n; fl1 = fl2n; abs1 = abs2n;
-    r0_2 = r0_3; nr2 = nr3;
   }
 }
 

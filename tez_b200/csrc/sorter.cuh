@@ -761,7 +761,7 @@ class SortPipeline {
           uint32_t grid = (uint32_t)std::min<uint64_t>(tiles, (uint64_t)num_sms * (per_sm > 0 ? per_sm : 1));
           k_emit_tma<<<grid, ET_THREADS, smem, stream>>>(fp, (uint32_t)EmitTmaLayout::stage_bytes(e.recs_per_tile, stride));
         } else if (fast_aligned && emit4_fits(e.recs_per_tile, fp.cpr) && !getenv("TEZGPU_EMIT_V2")) {
-          // software-pipelined kernel (emit_pipe.cuh): a tile's pieces must fit the registers of one gather round.
+          // software-pipelined kernel (emit_pipe.cuh): a tile's pieces must fit one stage of its gather ring.
           // Default: independent 256-thread CTAs, three per SM.  TEZGPU_EMIT_SUBS=3 selects the variant with one CTA
           // per SM whose three groups share lane-private checksum tables -- measured SLOWER (8.39 vs 5.44 ms): its
           // 219 KB of shared memory leave the SM ~30 KB of L1 and the random gather loses its memory-level parallelism.

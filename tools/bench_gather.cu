@@ -1,5 +1,6 @@
 // bench_gather.cu -- ceiling for the emit kernel's memory pattern: out[i] = in[perm[i]] for 80-byte records
 // (16-byte pieces, 5 lanes per record, streaming stores), no checksum, no framing.  Prints ms and GB/s moved.
+// Variants: LDG.128 into registers, per-thread cp.async (LDGSTS) into shared memory, bulk copies (TMA), cudaMemcpy.
 // build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/bench_gather tools/bench_gather.cu
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -170,6 +171,86 @@ static void run_tma(const uint8_t *in, const uint32_t *perm, uint8_t *out, uint3
   }
 }
 
+// ---------------------------------------------------------------------------------------------- LDGSTS (cp.async) variant
+// Per-thread asynchronous copies: each thread lands its 5 pieces of a 256-record tile with cp.async.cg (16 B, SASS
+// LDGSTS) in a thread-private ring of D stages (piece u of thread t in stage s at [s][u][t]), one commit group per
+// tile, and writes a tile out with LDS.128 + STG.128 once cp.async.wait_group D-1 says it landed.  No barriers: only
+// the issuing thread reads a slot.  The CTA's dynamic shared memory is padded to `smem` so that the run has the
+// occupancy and L1 carve-out of the emit kernel it models.
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void *src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+__device__ __forceinline__ uint4 lds_v4(uint32_t a) {
+  uint4 v;
+  asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
+  return v;
+}
+
+template <int D>
+__global__ void __launch_bounds__(256) k_gather_ldgsts(const uint8_t *__restrict__ in, const uint32_t *__restrict__ perm,
+                                                       uint8_t *__restrict__ out, uint32_t ntiles) {
+  extern __shared__ __align__(16) uint8_t smem[];
+  const uint32_t ring = smem_u32(smem) + 16u * threadIdx.x;  // + (s * 5 + u) * 4096
+  uint32_t tile = blockIdx.x;
+  // record indices of the next tile to issue, one tile ahead of the issue
+  uint32_t idx[5];
+  auto load_idx = [&](uint32_t t) {
+#pragma unroll
+    for (int u = 0; u < 5; u++) {
+      const uint32_t q = u * 256 + threadIdx.x, r = q / 5;
+      idx[u] = t < ntiles ? perm[(uint64_t)t * TILE_RECS + r] : 0u;
+    }
+  };
+  auto issue = [&](uint32_t t, int s) {
+    if (t < ntiles) {
+#pragma unroll
+      for (int u = 0; u < 5; u++) {
+        const uint32_t q = u * 256 + threadIdx.x, c = q - 5 * (q / 5);
+        cp_async16(ring + (s * 5 + u) * 4096u, in + (uint64_t)idx[u] * 80 + 16 * c);
+      }
+    }
+    cp_async_commit();  // empty groups past the end keep the group count per tile uniform
+  };
+  load_idx(tile);
+#pragma unroll
+  for (int s = 0; s < D; s++) {
+    const uint32_t t = tile + s * gridDim.x;
+    issue(t, s);
+    load_idx(t + gridDim.x);
+  }
+  for (int s = 0; tile < ntiles; tile += gridDim.x, s = s + 1 == D ? 0 : s + 1) {
+    cp_async_wait<D - 1>();
+    uint8_t *dst = out + (uint64_t)tile * TILE_BYTES + 16 * threadIdx.x;
+#pragma unroll
+    for (int u = 0; u < 5; u++) stg_stream_v4(dst + u * 4096, lds_v4(ring + (s * 5 + u) * 4096u));
+    const uint32_t t = tile + D * gridDim.x;
+    issue(t, s);
+    load_idx(t + gridDim.x);
+  }
+}
+
+template <int D>
+static void run_ldgsts(const uint8_t *in, const uint32_t *perm, uint8_t *out, uint32_t n, int ctas_per_sm, size_t smem,
+                       cudaEvent_t e0, cudaEvent_t e1) {
+  cudaFuncSetAttribute(k_gather_ldgsts<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  int per_sm = 0;
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_gather_ldgsts<D>, 256, smem);
+  const uint32_t ntiles = n / TILE_RECS;
+  for (int rep = 0; rep < 3; rep++) {
+    cudaEventRecord(e0);
+    k_gather_ldgsts<D><<<148 * ctas_per_sm, 256, smem>>>(in, perm, out, ntiles);
+    cudaEventRecord(e1);
+    cudaEventSynchronize(e1);
+    float ms;
+    cudaEventElapsedTime(&ms, e0, e1);
+    if (rep) printf("LDGSTS gather (cp.async.cg 16 B, thread-private ring), D = %d, %d CTAs/SM (%d resident), %.1f KB smem/CTA: %.3f ms, %.0f GB/s  [%s]\n",
+                    D, ctas_per_sm, per_sm, smem / 1024.0, ms, (double)n * 164 / (ms * 1e-3) / 1e9, cudaGetErrorString(cudaGetLastError()));
+  }
+}
+
 static void check_copy(const uint8_t *d_in, const uint32_t *d_perm, const uint8_t *d_out, uint32_t n) {
   // spot check: records 0, 1, n/2 of the output equal the permuted input
   uint32_t probe[3] = {0, 1, (n / 256) * 256 - 1};
@@ -203,7 +284,7 @@ int main(int argc, char **argv) {
   cudaEventCreate(&e0);
   cudaEventCreate(&e1);
   const uint64_t npieces = (uint64_t)n * 5;
-  for (int ctas = 2; ctas <= 8; ctas += 2) {
+  for (int ctas : {2, 3, 4, 6, 8}) {
     for (int rep = 0; rep < 2; rep++) {
       cudaEventRecord(e0);
       k_gather<5><<<148 * ctas, 256>>>(in, perm, out, npieces);
@@ -215,6 +296,20 @@ int main(int argc, char **argv) {
                       (double)n * 164 / (ms * 1e-3) / 1e9);
     }
   }
+  // LDGSTS variants, each at the shared-memory footprint k_emit_fast4 has with that ring (emit_pipe.cuh, Emit4Smem):
+  // 5120 B tables + 22016 B image + (D+1) KB indices + BATCH KB partials + 32 B per parked tile + (D+3) * 32 B
+  // descriptors + D * 20 KB ring.  Only the (CTAs/SM, D, BATCH) that fit 228 KB per SM (1 KB reserved per CTA).
+  auto fe4_smem = [](int d, int batch) { return (size_t)5120 + 22016 + (d + 1) * 1024 + batch * 1024 + batch * 32 + (d + 3) * 32 + d * 20480; };
+  cudaMemset(out, 0, (size_t)n * 80);
+  run_ldgsts<1>(in, perm, out, n, 2, fe4_smem(1, 8), e0, e1);
+  check_copy(in, perm, out, n);
+  run_ldgsts<2>(in, perm, out, n, 2, fe4_smem(2, 8), e0, e1);
+  run_ldgsts<3>(in, perm, out, n, 2, fe4_smem(3, 8), e0, e1);
+  run_ldgsts<1>(in, perm, out, n, 3, fe4_smem(1, 8), e0, e1);
+  cudaMemset(out, 0, (size_t)n * 80);
+  run_ldgsts<2>(in, perm, out, n, 3, fe4_smem(2, 4), e0, e1);
+  check_copy(in, perm, out, n);
+  run_ldgsts<1>(in, perm, out, n, 4, fe4_smem(1, 4), e0, e1);
   // TMA variants
   cudaMemset(out, 0, (size_t)n * 80);
   run_tma<4, 0, 1, 1>(in, perm, out, n, 2, e0, e1);
